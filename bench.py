@@ -24,6 +24,13 @@ replayed; time is CUDA events on the launching stream, max over ranks.
   cpu_baseline = the reference's own AVX2 kernels (oracle/_ref, built from /root/reference) on the
               box's host cores, bounded sample of the same workload
   --impl reference : that CPU arm alone, same metric / config.
+
+Inputs are seeded: the same arguments give the same weights and activations in every run.
+--dump-outputs DIR writes what the step computed in its last run as float32 .npy files, so that
+two builds can be compared output for output:
+  launch_chain.npy             [LAYERS][out]  one tmac_b200_gemv per layer, layer i on its own row x[i]
+  sequence_dependent_chain.npy [LAYERS][out]  the decode sequence (x[i+1] = first K outputs of layer i)
+(with N > 1 ranks: [ranks][LAYERS][out], the gathered outputs as rank 0 holds them)
 """
 import argparse
 import json
@@ -62,6 +69,17 @@ def synth(seed, mout=MOUT, k=K, bits=BITS, gs=GS, zp=ZP, one_scale=False):
     # alone the mean entry gives the 4096x4096 block a spectral radius of 16.6: 1e37 at layer 31, inf in some runs)
     z = (-0.5 * sc + rng.standard_normal((mout, k // gs)) * 0.001).astype(np.float16).astype(np.float32) if zp else None
     return w, sc, z
+
+
+def activations(seed, rows=LAYERS, k=K):
+    """Seeded fp16-representable activation rows, one per layer."""
+    return np.random.default_rng(seed).standard_normal((rows, k)).astype(np.float16).astype(np.float32)
+
+
+def dump_outputs(dirname, arrays):
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
 
 class ClockSampler:
@@ -234,7 +252,12 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-extras", action="store_true", help="skip tokens/s extras and the CPU baseline")
     ap.add_argument("--eager", action="store_true", help="no CUDA graph (for ncu kernel-level profiling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the step's last run to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU step's outputs; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -246,6 +269,7 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (no CPU fallback in the product path)")
+    torch.manual_seed(rank)                     # the inputs of the extras
     torch.cuda.set_device(local)
     dist = None
     force_sharded = os.environ.get("TMAC_BENCH_FORCE_SHARDED", "0") == "1"      # validate the N > 1 extras on one rank
@@ -268,7 +292,7 @@ def main():
     layers = [base] + [tb.clone(base) for _ in range(LAYERS - 1)]
     nag = K // AGS
     with torch.cuda.stream(stream):
-        x = torch.randn((LAYERS, K), device="cuda").half().float()
+        x = torch.from_numpy(activations(200 + rank)).cuda()
         qlut = torch.zeros((LAYERS, K // 4, 16), dtype=torch.int8, device="cuda")
         ls = torch.zeros((LAYERS, nag), device="cuda"); lb = torch.zeros_like(ls)
         out = torch.zeros((LAYERS, MOUT), device="cuda")
@@ -402,6 +426,8 @@ def main():
         sampler.start()
         time.sleep(0.3)
     ms = timed(g_step, args.steps, True)
+    # the outputs of the last timed step, before the replays below
+    dumps = {"launch_chain": (gathered if world > 1 else out).cpu().numpy()} if args.dump_outputs else {}
     launches["n"] = args.steps * kernels_per_step
     # keep the GPU busy a little longer so that the 100 ms clock sampler sees load
     t_end = time.time() + 1.0
@@ -461,7 +487,10 @@ def main():
     if "error" in seqs:
         seq_report = seqs
     else:
-        ms_dep, ms_ind, ms_sk = timed_seq(seqs["dependent"], args.steps, sv2), timed_seq(seqs["independent"], args.steps), timed_seq(seqs["dependent_streamk"], args.steps)
+        ms_dep = timed_seq(seqs["dependent"], args.steps, sv2)
+        if args.dump_outputs:
+            dumps["sequence_dependent_chain"] = (gathered2 if world > 1 else out_seq).cpu().numpy()
+        ms_ind, ms_sk = timed_seq(seqs["independent"], args.steps), timed_seq(seqs["dependent_streamk"], args.steps)
         seqs["dependent"].launch(); seqs["dependent"].status()       # the dependent chain's outputs for the parity check (host copy taken now)
         seq_gather_ok = None
         if world > 1:
@@ -496,6 +525,8 @@ def main():
             submission = "ONE persistent launch per step (%s); GEMV i+1 consumes GEMV i's output" % seq_kind.split(":")[0]
             step_is_sequence = resident
 
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumps)
     timed(g_two, 3, False)
     ms_two = timed(g_two, args.steps, False) / args.steps
     # ---- roofline of the dominant kernel: gemv launches only --------------------------------------
@@ -545,7 +576,7 @@ def main():
                                       "us_per_gemv": t_gr / LAYERS * 1e6, "launch": grouped_cfg}
 
     # ---- e2e: host buffers through the reference-facing call -----------------------------------
-    hx = torch.randn((LAYERS, K)).half().float().pin_memory()
+    hx = torch.from_numpy(activations(300 + rank)).pin_memory()
     hout = torch.zeros((LAYERS, MOUT)).pin_memory()
     hx_rows = [hx[i] for i in range(LAYERS)]          # the caller's per-layer host buffers (page-locked)
     hout_rows = [hout[i] for i in range(LAYERS)]
@@ -556,7 +587,7 @@ def main():
 
     for _ in range(3):
         e2e_step()
-    e2e_steps = max(3, min(args.steps, 20))
+    e2e_steps = args.steps
     if world > 1:
         dist.barrier()
     t0 = time.perf_counter()
