@@ -75,7 +75,8 @@ struct PinBuf {
 struct Resident {
     tmac_b200_kcfg cfg{};
     StreamLayout L{};
-    unsigned char *d = nullptr;          // stream layout in HBM
+    unsigned char *d = nullptr;          // stream layout in HBM, then the fp16 prefill tile's row exponents (int [nrsb * rsb] at rexp_off)
+    size_t rexp_off = 0, alloc = 0;      // offset of the row exponents, bytes allocated at d
     const unsigned char *host_a = nullptr;  // alias key: reference-layout host range
     size_t host_a_bytes = 0;
     int row0 = 0;                        // first row of the full tensor held here (row shards)
@@ -130,7 +131,7 @@ struct Context {
     std::set<const void *> sym_qluts;    // device QLUT buffers last written by our preprocessor
     std::vector<std::pair<std::vector<const void *>, void *>> ptr_tables;   // grouped-launch pointer tables
     // workspaces
-    DevBuf d_b, d_qlut, d_ls, d_lb, d_c, d_cbits, d_trace, d_tiles, d_pf_scratch, d_pf_flags;
+    DevBuf d_b, d_qlut, d_ls, d_lb, d_c, d_cbits, d_trace, d_tiles, d_pf_scratch, d_pf_flags, d_pf_texp;
     int trace = 0, trace_ctas = 0, trace_seq = 0;
     int chain_flags = 0;                 // resident chain (tmac_chain.cuh): bit 0 = grid-barrier form (comparison); default: data flow
     PinBuf h_in, h_out;
@@ -421,13 +422,27 @@ int launch_prefill(const Resident &R, int N, const int8_t *qlut, const float *ls
         const size_t smem16 = (size_t)kP16NA * kP16SubA + (size_t)kP16NB * kP16SubB + 2 * rawsz + (2 * kP16NA + 2 * kP16NB + 2) * 8 + 1024;
         if (smem16 <= 227 * 1024) {
             if (g.d_tiles.ensure((size_t)ntile16 * (nmain + nextra) * kP16BBytes)) return fail("out of device memory (LUT tiles)");
-            lut_tile16_kernel<<<dim3(nmain + nextra, ntile16), 256, 0, g.stream()>>>(qlut, ls, lb, (unsigned char *)g.d_tiles.p, N, L.K, nmain, nextra);
-            CUDA_OK(cudaGetLastError());
+            if (g.d_pf_texp.ensure((size_t)N * sizeof(int))) return fail("out of device memory (token exponents)");
+            {   // programmatic dependent launches: the exponent scan starts under the preprocessor's tail, the tiling kernel loads its
+                // LUT entries while the exponents are being computed (each waits on griddepcontrol before it reads its inputs)
+                cudaLaunchConfig_t lc{};
+                lc.blockDim = dim3(256); lc.stream = g.stream();
+                cudaLaunchAttribute at[1];
+                at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+                at[0].val.programmaticStreamSerializationAllowed = g.use_pdl ? 1 : 0;
+                lc.attrs = at; lc.numAttrs = 1;
+                lc.gridDim = dim3((N + 7) / 8);
+                CUDA_OK(cudaLaunchKernelEx(&lc, p16_token_exp_kernel, ls, lb, (int *)g.d_pf_texp.p, N, nmain));
+                lc.gridDim = dim3(nmain + nextra, ntile16);
+                CUDA_OK(cudaLaunchKernelEx(&lc, lut_tile16_kernel, qlut, ls, lb, (const int *)g.d_pf_texp.p, (unsigned char *)g.d_tiles.p,
+                                           N, (int)L.K, nmain, nextra));
+            }
             Prefill16Params q{};
             q.W = R.d; q.C = C; q.N = N; q.K = L.K; q.Mout = L.Mout; q.ldc = ldc; q.out_f16 = out_f16;
             q.nchunk = L.nchunk; q.zp = L.zp; q.sd = L.sd; q.blk_bytes = (int)L.blk; q.nmain = nmain; q.nextra = nextra;
             q.rsb_stride = L.rsb_stride; q.tiles = (const unsigned char *)g.d_tiles.p;
             q.nrsb = L.nrsb; q.ntiles = L.nrsb * ntile16;
+            q.texp = (const int *)g.d_pf_texp.p; q.rexp = reinterpret_cast<const int *>(R.d + R.rexp_off);
             // fewer tiles than SMs (e.g. 86 at N = 256): stream-K over all SMs, partial tiles through `scratch`
             q.streamk = (g.pf_streamk && q.ntiles < g.sms && (long)q.ntiles * (nmain + nextra) >= 2L * g.sms) ? 1 : 0;
             const int grid = q.streamk ? g.sms : q.ntiles;
@@ -545,12 +560,20 @@ int64_t register_resident(const tmac_b200_kcfg &cfg, const PlainWeights &P, cons
     if (!make_layout(P.Mout, cfg.K, cfg.bits, cfg.group_size, cfg.act_group_size, cfg.zero_point, cfg.one_scale, fp16_ok ? 2 : 4, &L))
         return fail("unsupported shape / grouping for the stream layout");
     if (cfg.one_scale) L.scale0 = P.scales.empty() ? 0.f : P.scales[0];
-    std::vector<uint8_t> host(L.total);
-    encode_stream(P, L, host.data());
     Resident R;
+    R.rexp_off = (L.total + 15) & ~(size_t)15;
+    R.alloc = R.rexp_off + (size_t)L.nrsb * L.rsb * sizeof(int);
+    std::vector<uint8_t> host(R.alloc, 0);
+    encode_stream(P, L, host.data());
+    if (!cfg.one_scale) {                // per-row exponents of the fp16 prefill tile (tmac_prefill16.cuh, p16_exp); padding rows 0
+        const int ng = cfg.K / cfg.group_size;
+        int *rexp = reinterpret_cast<int *>(host.data() + R.rexp_off);
+        for (int r = 0; r < P.Mout; ++r)
+            rexp[r] = p16_row_exp(P.scales.data() + (size_t)r * ng, P.zeros.empty() ? nullptr : P.zeros.data() + (size_t)r * ng, ng);
+    }
     R.cfg = cfg; R.L = L; R.row0 = row0;
-    if (cudaMalloc((void **)&R.d, L.total) != cudaSuccess) { cudaGetLastError(); return fail("out of device memory for resident weights"); }
-    if (cudaMemcpy(R.d, host.data(), L.total, cudaMemcpyHostToDevice) != cudaSuccess) { cudaFree(R.d); return fail("weight upload failed"); }
+    if (cudaMalloc((void **)&R.d, R.alloc) != cudaSuccess) { cudaGetLastError(); return fail("out of device memory for resident weights"); }
+    if (cudaMemcpy(R.d, host.data(), R.alloc, cudaMemcpyHostToDevice) != cudaSuccess) { cudaFree(R.d); return fail("weight upload failed"); }
     R.host_a = (const unsigned char *)host_alias;
     R.host_a_bytes = alias_bytes;
     const int64_t h = g.next_handle++;
@@ -632,7 +655,7 @@ void tmac_b200_shutdown(void) {
         std::free(kv.second.host_scales);
     }
     g.res.clear();
-    for (DevBuf *b : {&g.d_b, &g.d_qlut, &g.d_ls, &g.d_lb, &g.d_c, &g.d_cbits, &g.d_trace, &g.d_tiles, &g.d_pf_scratch, &g.d_pf_flags}) { if (b->p) cudaFree(b->p); b->p = nullptr; b->cap = 0; }
+    for (DevBuf *b : {&g.d_b, &g.d_qlut, &g.d_ls, &g.d_lb, &g.d_c, &g.d_cbits, &g.d_trace, &g.d_tiles, &g.d_pf_scratch, &g.d_pf_flags, &g.d_pf_texp}) { if (b->p) cudaFree(b->p); b->p = nullptr; b->cap = 0; }
     for (HostLut &e : g.hluts) {
         for (DevBuf *b : {&e.dq, &e.dls, &e.dlb}) { if (b->p) cudaFree(b->p); b->p = nullptr; b->cap = 0; }
         if (e.res.p) cudaFreeHost(e.res.p);
@@ -882,8 +905,8 @@ int64_t tmac_b200_clone_weights(int64_t handle) {
     Resident R = it->second;
     R.host_a = nullptr; R.host_a_bytes = 0;
     R.reserved = nullptr; R.reserved_bytes = 0; R.host_scales = nullptr;   // owned by the original only (no double munmap / free)
-    if (cudaMalloc((void **)&R.d, R.L.total) != cudaSuccess) { cudaGetLastError(); return fail("out of device memory for clone"); }
-    if (cudaMemcpy(R.d, it->second.d, R.L.total, cudaMemcpyDeviceToDevice) != cudaSuccess) { cudaFree(R.d); return fail("clone copy failed"); }
+    if (cudaMalloc((void **)&R.d, R.alloc) != cudaSuccess) { cudaGetLastError(); return fail("out of device memory for clone"); }
+    if (cudaMemcpy(R.d, it->second.d, R.alloc, cudaMemcpyDeviceToDevice) != cudaSuccess) { cudaFree(R.d); return fail("clone copy failed"); }
     const int64_t h = g.next_handle++;
     R.id = h;
     g.res[h] = R;

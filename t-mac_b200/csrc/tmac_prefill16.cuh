@@ -9,9 +9,10 @@
 // ride in the operands: A = fp16(0.5*s*S) is expanded by the producers from the packed codes, B = fp16(ls*T8) is laid out
 // once per call by lut_tile16_kernel, the accumulator lives in TMEM for the whole K and is read once.  The bias term is one
 // more contraction step with exact operands: A columns (0.5s, 0.5s, z, z) against B columns (LBhi, LBlo, LBhi, LBlo), LB
-// split into two fp16 so that their sum carries 22 bits.  Operand rounding (2^-11 per B entry) keeps the result inside
-// north_star's 1e-3 of the CPU kernel (tools/sim_fp16_prefill.py: 1.4e-4 W2, 2.4e-4 W4) -- NOT inside the 2e-5 the exact
-// paths hold, so this tile has its own tolerance and never serves the int32 (BitNet) path.
+// split into two fp16 so that their sum carries 22 bits.  Both operands are normalised per token and per row by powers of two
+// (see p16_exp below), so fp16's range never clips them.  Operand rounding (2^-11 per entry) keeps every output within
+// 2.5e-4 x sum_k |x_k| |W_mk| of the CPU kernel -- NOT inside the 2e-5 the exact paths hold, so this tile has its own
+// tolerance and never serves the int32 (BitNet) path.
 //
 // Tile: 128 weight rows x 256 tokens per CTA, tcgen05.mma kind::f16 (M 128, N 256, K 16), 8 MMAs per activation group.
 //   warps 0..15 : producers (thread = weight row x 4 of the step's 16 groups): code byte -> 8 unit fp16 from a 256-entry
@@ -44,7 +45,50 @@ struct Prefill16Params {
     int nrsb, ntiles, streamk;                       // row super-blocks, tiles = nrsb * token tiles, stream-K split (see the kernel)
     float *scratch;                                  // [grid][256 tokens][128 rows] fp32 partial tiles (stream-K)
     int *flags;                                      // [grid] partial tile ready
+    const int *texp;                                 // [N] token exponents e_n (p16_token_exp_kernel)
+    const int *rexp;                                 // [nrsb * 128] row exponents f_m (p16_row_exp, computed at upload)
 };
+
+// Range handling.  fp16 holds 2^-14 .. 65504 at full precision, the inputs do not come in that range: a token's LUT biases
+// reach 128 x its activations (inf past 65504), small scales or activations fall into fp16's subnormals.  So both operands are
+// normalised by exact powers of two: token n's B entries and biases by 2^-e_n (its largest entry lands in [2^14, 2^15)), row
+// m's 0.5*scale and zero by 2^-f_m (largest in [2^13, 2^14), so that the A entry 3 * 0.5*scale stays below 65504); the
+// epilogue multiplies by 2^(e_n + f_m).  Scaling a token or a row by 2^k then shifts e_n or f_m by k and leaves every operand
+// bit unchanged: the tile's output scales by exactly 2^k, as the exact paths' does.  Exponents are clamped to +-64 so that every
+// factor 2^e is an fp32 normal and the epilogue's val * 2^e_n * 2^f_m is exact (|val| < 2^47 after normalisation); the clamp
+// binds only for token or row magnitudes beyond 2^+-49.
+__host__ __device__ inline int p16_exp(float m, int top) {   // e with m * 2^-e in [2^(top-1), 2^top); 0 for 0, inf, NaN
+    if (!(m > 0.f) || m > 3.4e38f) return 0;
+    int e;
+    frexpf(m, &e);
+    return e - top < -64 ? -64 : (e - top > 64 ? 64 : e - top);
+}
+
+__device__ __forceinline__ float p16_pow2(int e) { return __int_as_float((e + 127) << 23); }   // 2^e, -126 <= e <= 127
+
+inline int p16_row_exp(const float *scales, const float *zeros, int ng) {     // f_m of one row: ng groups
+    float m = 0.f;
+    for (int g = 0; g < ng; ++g) {
+        m = std::max(m, 0.5f * std::fabs(scales[g]));
+        if (zeros) m = std::max(m, std::fabs(zeros[g]));
+    }
+    return p16_exp(m, 14);
+}
+
+// e_n of every token: one warp per token scans its K/64 LUT scales and K/128 bias pairs (the same sums lut_tile16_kernel forms).
+__global__ void __launch_bounds__(256) p16_token_exp_kernel(const float *ls, const float *lb, int *texp, int N, int nag) {
+    const int n = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    pdl_wait();                                      // ls / lb: the preprocessor (or the caller's work) before this launch
+    pdl_launch_dependents();                         // lut_tile16_kernel loads its LUT entries meanwhile, then waits for texp
+    if (n >= N) return;
+    const float *l = ls + (size_t)n * nag, *b = lb + (size_t)n * nag;
+    float m = 0.f;
+    for (int i = lane; i < nag; i += 32) m = fmaxf(m, 128.f * fabsf(l[i]));
+    for (int i = lane; i < nag / 2; i += 32) m = fmaxf(m, fabsf(b[2 * i] + b[2 * i + 1]));
+#pragma unroll
+    for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if (lane == 0) texp[n] = p16_exp(m, 15);
+}
 
 __device__ __forceinline__ uint64_t p16_desc(uint32_t saddr, uint32_t lbo) {
     uint64_t d = (uint64_t)((saddr >> 4) & 0x3FFF);
@@ -55,24 +99,28 @@ __device__ __forceinline__ uint64_t p16_desc(uint32_t saddr, uint32_t lbo) {
 }
 
 // B tiles.  grid = (nmain + nextra, token tiles of 256), block = 256 (thread = token).
-//   step < nmain : entries (lut_scale[n][step] * T8[n][16*step + g][e]) as fp16, token t, group g at ((g*32 + t/8)*128 + (t%8)*16)
-//   bias steps   : column 4*wg + {0,1,2,3} = {LBhi, LBlo, LBhi, LBlo}, LB = lut_bias[n][2wg] + lut_bias[n][2wg+1]; 8 columns per chunk
-__global__ void __launch_bounds__(256) lut_tile16_kernel(const int8_t *qlut, const float *ls, const float *lb, unsigned char *out, int N, int K,
-                                                         int nmain, int nextra) {
+//   step < nmain : entries (lut_scale[n][step] * 2^-e_n * T8[n][16*step + g][e]) as fp16, token t, group g at ((g*32 + t/8)*128 + (t%8)*16)
+//   bias steps   : column 4*wg + {0,1,2,3} = {LBhi, LBlo, LBhi, LBlo}, LB = (lut_bias[n][2wg] + lut_bias[n][2wg+1]) * 2^-e_n; 8 columns per chunk
+__global__ void __launch_bounds__(256) lut_tile16_kernel(const int8_t *qlut, const float *ls, const float *lb, const int *texp, unsigned char *out,
+                                                         int N, int K, int nmain, int nextra) {
     const int step = blockIdx.x, tile = blockIdx.y, t = threadIdx.x, n = tile * kP16NT + t;
     const int nag = K / 64, nwg = K / 128;
     unsigned char *rec = out + ((size_t)tile * (nmain + nextra) + step) * kP16BBytes;
     if (step < nmain) {
-        const float l = (n < N) ? ls[(size_t)n * nag + step] : 0.f;
         const uint2 *src = reinterpret_cast<const uint2 *>(qlut) + ((size_t)n * (K / 4) + (size_t)step * 16) * 2;
+        uint2 q[16];
+        float l = 0.f;
+#pragma unroll
+        for (int g = 0; g < 16; ++g) q[g] = (n < N) ? __ldg(src + g * 2) : make_uint2(0, 0);   // the 8 stored entries of each group
+        if (n < N) l = ls[(size_t)n * nag + step];
+        pdl_wait();                                  // texp: p16_token_exp_kernel, launched just before as the primary grid
+        if (n < N) l *= p16_pow2(-texp[n]);
 #pragma unroll
         for (int g = 0; g < 16; ++g) {
-            uint2 q = make_uint2(0, 0);
-            if (n < N) q = __ldg(src + g * 2);       // the 8 stored entries of the group
             uint32_t o[4];
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-                const uint32_t word = k < 2 ? q.x : q.y;
+                const uint32_t word = k < 2 ? q[g].x : q[g].y;
                 const float a = (float)(int)(int8_t)((word >> (16 * (k & 1))) & 0xff) * l;
                 const float b = (float)(int)(int8_t)((word >> (16 * (k & 1) + 8)) & 0xff) * l;
                 const __half2 h = __floats2half2_rn(a, b);
@@ -82,6 +130,8 @@ __global__ void __launch_bounds__(256) lut_tile16_kernel(const int8_t *qlut, con
         }
     } else {
         const int e = step - nmain;                  // bias step: weight groups 32e .. 32e+31, two per 16-byte chunk
+        pdl_wait();
+        const float sn = p16_pow2((n < N) ? -texp[n] : 0);
 #pragma unroll
         for (int kc = 0; kc < 16; ++kc) {
             uint32_t o[4];
@@ -89,7 +139,7 @@ __global__ void __launch_bounds__(256) lut_tile16_kernel(const int8_t *qlut, con
             for (int u = 0; u < 2; ++u) {
                 const int wg = e * 32 + kc * 2 + u;
                 float LB = 0.f;
-                if (n < N && wg < nwg) LB = lb[(size_t)n * nag + 2 * wg] + lb[(size_t)n * nag + 2 * wg + 1];
+                if (n < N && wg < nwg) LB = (lb[(size_t)n * nag + 2 * wg] + lb[(size_t)n * nag + 2 * wg + 1]) * sn;
                 const __half hi = __float2half_rn(LB);
                 const __half lo = __float2half_rn(LB - __half2float(hi));
                 const __half2 h = __halves2half2(hi, lo);
@@ -117,6 +167,7 @@ __global__ void __launch_bounds__(kP16Threads, 1) prefill16_w2_kernel(const Pref
     uint64_t *bars = reinterpret_cast<uint64_t *>(raw + 2 * rawsz);
     uint64_t *fullA = bars, *emptyA = fullA + kP16NA, *fullB = emptyA + kP16NA, *emptyB = fullB + kP16NB, *accfull = emptyB + kP16NB;   // accfull[2]
     __shared__ uint32_t tmem_base_s;
+    __shared__ float tok_scale[2][kP16NT];                                  // 2^e_n of each fragment's tokens (epilogue)
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int nsteps = p.nmain + p.nextra;
@@ -155,6 +206,8 @@ __global__ void __launch_bounds__(kP16Threads, 1) prefill16_w2_kernel(const Pref
         for (int f = 0; f < nfrag; ++f) {
             const int rsb = ft[f] % p.nrsb;
             const unsigned char *rsb_base = p.W + (size_t)rsb * p.rsb_stride;
+            const int f_m = p.rexp[rsb * 128 + r];
+            const float zsc = p16_pow2(-f_m), hsc = 0.5f * zsc;           // z * 2^-f_m, 0.5 * scale * 2^-f_m: exact
             const int s0 = fs0[f], s1m = min(fs1[f], p.nmain);
             if (s0 < s1m) {
                 const int c_first = s0 >> 1, c_last = (s1m - 1) >> 1;
@@ -173,8 +226,8 @@ __global__ void __launch_bounds__(kP16Threads, 1) prefill16_w2_kernel(const Pref
                     }
                     const uint32_t *words = reinterpret_cast<const uint32_t *>(rb);
                     // the row's 8 A entries of one K-group: +-hs at entry j0 (plane 0) plus +-2hs at entry j1 (plane 1), hs = fp16(0.5 * scale),
-                    // built in registers: (+-hs) + (+-2hs) is one fp16 rounding of the exact k * hs
-                    const __half hsh = __float2half_rn(0.5f * load_scale(rb + 4096, p.sd, wl * 4 + wi));
+                    // built in registers: (+-hs) + (+-2hs) is one fp16 rounding of the exact k * hs; hs = fp16(0.5 * scale * 2^-f_m)
+                    const __half hsh = __float2half_rn(load_scale(rb + 4096, p.sd, wl * 4 + wi) * hsc);
                     const uint32_t c1 = __half_as_ushort(hsh), c2 = __half_as_ushort(__hadd(hsh, hsh));
                     const int u0 = (c == c_first) ? (s0 & 1) : 0, u1 = (c == c_last) ? ((s1m - 1) & 1) : 1;   // steps of this chunk
 #pragma unroll 1
@@ -224,8 +277,8 @@ __global__ void __launch_bounds__(kP16Threads, 1) prefill16_w2_kernel(const Pref
                             float hs = 0.f, zz = 0.f;
                             if (wg < p.nchunk) {
                                 const unsigned char *sp = rsb_base + (size_t)wg * p.blk_bytes + 4096;
-                                hs = 0.5f * load_scale(sp, p.sd, wl * 4 + wi);
-                                if (p.zp) zz = load_scale(sp + (size_t)128 * p.sd, p.sd, wl * 4 + wi);
+                                hs = load_scale(sp, p.sd, wl * 4 + wi) * hsc;
+                                if (p.zp) zz = load_scale(sp + (size_t)128 * p.sd, p.sd, wl * 4 + wi) * zsc;
                             }
                             const __half2 a = __floats2half2_rn(hs, hs), b = __floats2half2_rn(zz, zz);
                             o[2 * u] = *reinterpret_cast<const uint32_t *>(&a); o[2 * u + 1] = *reinterpret_cast<const uint32_t *>(&b);
@@ -243,12 +296,18 @@ __global__ void __launch_bounds__(kP16Threads, 1) prefill16_w2_kernel(const Pref
         // partial tiles first (another CTA waits for them), then the tile this CTA finishes
         const int lq = warp & 3, cg = warp >> 2;     // TMEM lane quarter of this warp, columns 64*cg .. 64*cg+63
         const int er = lq * 32 + lane;
+        for (int i = tid; i < nfrag * kP16NT; i += kP16ProdWarps * 32) {
+            const int fi = i / kP16NT, n = ((fi ? ft[1] : ft[0]) / p.nrsb) * kP16NT + i % kP16NT;   // (no dynamic index: ft stays in registers)
+            tok_scale[fi][i % kP16NT] = p16_pow2(n < p.N ? p.texp[n] : 0);
+        }
+        asm volatile("bar.sync 1, 512;" ::: "memory");
         for (int pass = 0; pass < 2; ++pass)
             for (int f = 0; f < nfrag; ++f) {
                 const bool whole = fs0[f] == 0 && fs1[f] == nsteps, last = fs1[f] == nsteps;
                 if ((pass == 0) == last) continue;   // pass 0: fragments that do not hold the tile's last step
                 const int rsb = ft[f] % p.nrsb, tile = ft[f] / p.nrsb, n0 = tile * kP16NT, ntok = min(kP16NT, p.N - n0);
-                const int row = rsb * 128 + er;
+                const int row = rsb * 128 + er, f_m = p.rexp[row];
+                const float rf = p16_pow2(f_m);
                 pf_mbar_wait(accfull + f, 0);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 int c_first = cta;
@@ -283,6 +342,7 @@ __global__ void __launch_bounds__(kP16Threads, 1) prefill16_w2_kernel(const Pref
                             val = acc + val;
                         }
                         if (t < ntok && row < p.Mout) {
+                            val = val * tok_scale[f][t] * rf;   // undo the normalisation (exact, see p16_exp)
                             const size_t o = (size_t)(n0 + t) * p.ldc + row;
                             if (p.out_f16) reinterpret_cast<__half *>(p.C)[o] = __float2half_rn(val);
                             else reinterpret_cast<float *>(p.C)[o] = val;
